@@ -28,6 +28,15 @@ Numbers on the JSON line:
              scipy.fft, SSQ_PARALLEL=1 on all host cores, reused Wavelet, warm JIT) on a bounded
              sample of the same workload: one signal per step.  Falls back to the oracle port
              (kind "port") only if the package cannot be imported.
+
+`--dump-outputs DIR` writes what the last timed step computed, Tx.npy and Wx.npy (rank 0's
+shard on several GPUs), so that two builds can be compared output for output: the inputs are
+the same seeded chirps on every run.  A complex array is stored as its real view (float32 or
+float64, trailing axis of 2: real, imaginary); one larger than DUMP_BYTES / 2 is stored as a
+fixed sample of its flattened elements (one per stride, seeded offset within each stride:
+`dump_index`), so the files stay below 64 MB in all.  Wx repeats bit for bit from run to run;
+the fused reassignment adds into Tx with atomics, so Tx's last bits follow the summation order
+and two runs agree only to rounding (DESIGN section 2: bins exact, Tx <= 2e-6 norm-wise).
 """
 import argparse
 import json
@@ -50,6 +59,7 @@ CONFIGS = {
     'C5': (('gmw', {'beta': 12, 'gamma': 3, 'dtype': 'float64'}), 'float64', 1 << 20, 512, None, 'weak'),
 }
 FP32_PEAK_TFLOPS = 75.0          # 148 SMs x 128 FMA lanes x 2 x 1.965 GHz (CUDA cores, nominal)
+DUMP_BYTES = 60_000_000          # --dump-outputs: all files together (Tx and Wx, headers aside)
 
 
 def config_dict(name):
@@ -141,6 +151,28 @@ def log_scales(cwt_scalebounds, wavelet, N, na):
     nv = int(np.ceil(na / np.log2(mx / mn)))
     p0 = int(np.floor(nv * np.log2(mn)))
     return 2 ** (np.arange(p0, p0 + na) / nv)
+
+
+def dump_index(total, n, seed=0):
+    """Sorted flat indices of a fixed sample of n out of `total` elements: one in each of n equal
+    strides, at a seeded offset.  None when n covers them all."""
+    if total <= n:
+        return None
+    stride = total // n
+    return np.arange(n, dtype=np.int64) * stride + np.random.default_rng(seed).integers(0, stride, n)
+
+
+def output_arrays(outs, budget=DUMP_BYTES):
+    """{name: float array on the host} of complex device tensors, sampled by `dump_index` to share
+    `budget` bytes evenly."""
+    import torch
+    res = {}
+    for name, t in outs.items():
+        idx = dump_index(t.numel(), budget // len(outs) // t.element_size())
+        if idx is not None:
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        res[name] = torch.view_as_real(t).cpu().numpy()
+    return res
 
 
 def bind_to_gpu_numa(local_rank):
@@ -363,6 +395,7 @@ def run_b200(args):
 
     sampler = ClockSampler(local) if rank == 0 else None
     ms_per_step, launches = timed_steps(w, args.steps, args.warmup, world, dist, sampler)
+    dumped = output_arrays({'Tx': w.Tx, 'Wx': w.Wx}) if args.dump_outputs and rank == 0 else None
     if rank == 0:
         # the timed region can be shorter than nvidia-smi's sampling period: keep the same step
         # loop running for another 0.5 s so the clocks line has enough samples
@@ -517,6 +550,10 @@ def run_b200(args):
             "e2e_ridges": e2e_ridges, "gather_ms": gather_ms, "roofline": roofline, "c2": c2}
     if cpu is not None:
         line["cpu_baseline"] = {k: cpu[k] for k in ("value", "unit", "cores", "kind", "sample")}
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
     emit_line(line)
     if world > 1:
         dist.barrier()
@@ -557,7 +594,13 @@ def main():
     ap.add_argument('--gather', action='store_true', help='also time an NCCL all_gather of Tx')
     ap.add_argument('--no-ridges', dest='ridges', action='store_false',
                     help='skip the e2e variant that returns ridges instead of planes')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write Tx, Wx of the last timed step to DIR/<name>.npy (b200 only)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
     if args.warmup < 3 and args.impl == 'b200':
         args.warmup = 3
     if args.impl == 'reference':
