@@ -69,11 +69,7 @@ struct Gfft {
     A.R = R;
     size_t smem = ((size_t)2 * S.n * R + S.n) * sizeof(cx<T>);
     auto kern = gfft_smem_kernel<T>;
-    static size_t attr = 0;
-    if (smem > attr) {
-      SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      attr = smem;
-    }
+    SSQB_CUDA(set_smem_limit(kern, smem));
     kern<<<(unsigned)((count + R - 1) / R), 256, smem, st>>>(A);
     SSQB_LAUNCH_CHECK();
     return 0;

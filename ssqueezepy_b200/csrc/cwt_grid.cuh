@@ -291,7 +291,7 @@ template <typename T, int K, int PPK> struct InterpGeom {
   static constexpr int NT = 256;
 };
 
-template <typename T, int K, int PPK, int NARR, bool SSQ, bool REGWIN>
+template <typename T, int K, int PPK, int NARR, bool SSQ>
 __global__ void __launch_bounds__(256, (sizeof(T) == 4) ? 3 : 1)
 grid_interp_kernel(const GridArgs<T> G) {
   constexpr int PP = K * PPK;
@@ -403,38 +403,23 @@ grid_interp_kernel(const GridArgs<T> G) {
     }
   };
 
-  if constexpr (REGWIN) {
-    // register-resident sliding window
-    V4 win[K];
+  // register-resident sliding window
+  V4 win[K];
 #pragma unroll
-    for (int k = 0; k < K - 1; ++k) win[k] = Vs[wl0 + k];
+  for (int k = 0; k < K - 1; ++k) win[k] = Vs[wl0 + k];
 #pragma unroll 1
-    for (int g = 0; g < PPK; ++g) {
-      if (g * K >= np) break;
+  for (int g = 0; g < PPK; ++g) {
+    if (g * K >= np) break;
 #pragma unroll
-      for (int kk = 0; kk < K; ++kk) {
-        const int i = g * K + kk;
-        win[(kk + K - 1) % K] = Vs[wl0 + i + K - 1];
-        cx<T> aw = cscale<T>(mkc<T>(win[kk % K].x, win[kk % K].y), h[0]);
-        cx<T> ad = mkc<T>((T)0, (T)0);
-        if (NARR == 2) ad = cscale<T>(mkc<T>(win[kk % K].z, win[kk % K].w), h[0]);
+    for (int kk = 0; kk < K; ++kk) {
+      const int i = g * K + kk;
+      win[(kk + K - 1) % K] = Vs[wl0 + i + K - 1];
+      cx<T> aw = cscale<T>(mkc<T>(win[kk % K].x, win[kk % K].y), h[0]);
+      cx<T> ad = mkc<T>((T)0, (T)0);
+      if (NARR == 2) ad = cscale<T>(mkc<T>(win[kk % K].z, win[kk % K].w), h[0]);
 #pragma unroll
-        for (int k = 1; k < K; ++k) {
-          const V4 v = win[(kk + k) % K];
-          aw = caxpy<T>(mkc<T>(v.x, v.y), h[k], aw);
-          if (NARR == 2) ad = caxpy<T>(mkc<T>(v.z, v.w), h[k], ad);
-        }
-        emit(i, aw, ad);
-      }
-    }
-  } else {
-    // taps straight from shared memory (K x 32 bytes per output in float64: shared-memory bound)
-#pragma unroll 1
-    for (int i = 0; i < np; ++i) {
-      cx<T> aw = mkc<T>((T)0, (T)0), ad = mkc<T>((T)0, (T)0);
-#pragma unroll
-      for (int k = 0; k < K; ++k) {
-        const V4 v = Vs[wl0 + i + k];
+      for (int k = 1; k < K; ++k) {
+        const V4 v = win[(kk + k) % K];
         aw = caxpy<T>(mkc<T>(v.x, v.y), h[k], aw);
         if (NARR == 2) ad = caxpy<T>(mkc<T>(v.z, v.w), h[k], ad);
       }

@@ -34,11 +34,7 @@ static int launch_pass1_t(const CwtArgs<T>& A, int narr, cudaStream_t st) {
   constexpr int R1 = Tile<T>::ELEMS / M;
   size_t smem = ((size_t)M * (R1 + 1) + M) * sizeof(cx<T>);
   auto kern = cwt_pass1_kernel<T, LOG_M, MODE>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
+  SSQB_CUDA(set_smem_limit(kern, smem));
   long long ncol1 = (long long)A.nrows << A.logF;
   dim3 grid((unsigned)((ncol1 + R1 - 1) / R1), (unsigned)narr);
   kern<<<grid, Tile<T>::NT, smem, st>>>(A);
@@ -64,11 +60,7 @@ static int launch_pass2_t(const CwtArgs<T>& A, int write_dWx, cudaStream_t st) {
   constexpr int R2 = Tile<T>::ELEMS / F;
   size_t smem = ((size_t)NARR * Tile<T>::ELEMS + F) * sizeof(cx<T>);
   auto kern = cwt_pass2_kernel<T, LOG_F, NARR, EPI>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
+  SSQB_CUDA(set_smem_limit(kern, smem));
   long long ncols = (long long)A.nrows << A.logI2;
   dim3 grid((unsigned)((ncols + R2 - 1) / R2));
   kern<<<grid, Tile<T>::NT, smem, st>>>(A, write_dWx);
@@ -87,10 +79,14 @@ static int launch_pass2(const CwtArgs<T>& A, int write_dWx, cudaStream_t st) {
   }
 }
 
-static int g_rows_bpt = 1;     // butterflies per thread in the row kernels (SSQB_BPT=1|2)
+// cwt_rows_kernel: every row tile is 2^ROWS_LOGE points -- direct rows, block rows and pass 2 of
+// the two-pass rows (R2 = 8 lanes at F = 512).  One butterfly per thread in float32, two in
+// float64 (1024-thread CTAs need <= 64 registers).
+static constexpr int ROWS_LOGE = 12;
 
-template <typename T, int LOGE, int LOG_F, int NARR, int GEN, int QMAX, bool SSQ, int BPT>
-static int launch_rows_b(const FastArgs<T>& P, unsigned grid_y, cudaStream_t st) {
+template <typename T, int LOG_F, int NARR, int GEN, int QMAX>
+static int launch_rows(const FastArgs<T>& P, unsigned grid_y, cudaStream_t st) {
+  constexpr int LOGE = ROWS_LOGE, BPT = sizeof(T) == 4 ? 1 : 2;
   constexpr int ELEMS = 1 << LOGE;
   constexpr int NT = ELEMS / (8 * BPT);
   constexpr int F = 1 << LOG_F;
@@ -98,12 +94,10 @@ static int launch_rows_b(const FastArgs<T>& P, unsigned grid_y, cudaStream_t st)
   size_t smem = (size_t)512 * sizeof(cx<T>);
   if (LOG_F > 3) smem += (size_t)NARR * RowsTile<T, LOGE, LOG_F>::SARR * sizeof(cx<T>);
   if (GEN == GEN_DIRECT) smem += (size_t)QMAX * F * 4 * sizeof(T);
-  auto kern = cwt_rows_kernel<T, LOGE, LOG_F, NARR, GEN, QMAX, SSQ, BPT>;
-  static size_t attr_smem = 0;
-  if (smem > attr_smem) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_smem = smem;
-  }
+  auto kern = cwt_rows_kernel<T, LOGE, LOG_F, NARR, GEN, QMAX, false, BPT>;
+  if constexpr (NARR == 2)
+    if (P.ssq) kern = cwt_rows_kernel<T, LOGE, LOG_F, 2, GEN, QMAX, true, BPT>;
+  SSQB_CUDA(set_smem_limit(kern, smem));
   long long nF = (long long)A.n_up >> LOG_F;         // output phases per row
   dim3 grid((unsigned)(nF / (ELEMS / F)), grid_y);
   kern<<<grid, NT, smem, st>>>(P);
@@ -111,109 +105,67 @@ static int launch_rows_b(const FastArgs<T>& P, unsigned grid_y, cudaStream_t st)
   return 0;
 }
 
-template <typename T, int LOGE, int LOG_F, int NARR, int GEN, int QMAX, bool SSQ>
-static int launch_rows_s(const FastArgs<T>& P, unsigned grid_y, cudaStream_t st) {
-  // 1024-thread CTAs need <= 64 registers: float32 only
-  if (g_rows_bpt == 1 && sizeof(T) == 4)
-    return launch_rows_b<T, LOGE, LOG_F, NARR, GEN, QMAX, SSQ, 1>(P, grid_y, st);
-  return launch_rows_b<T, LOGE, LOG_F, NARR, GEN, QMAX, SSQ, 2>(P, grid_y, st);
-}
-
-template <typename T, int LOGE, int LOG_F, int NARR, int GEN, int QMAX>
-static int launch_rows_t(const FastArgs<T>& P, unsigned grid_y, cudaStream_t st) {
-  if (NARR == 2 && P.ssq)
-    return launch_rows_s<T, LOGE, LOG_F, 2, GEN, QMAX, true>(P, grid_y, st);
-  return launch_rows_s<T, LOGE, LOG_F, NARR, GEN, QMAX, false>(P, grid_y, st);
-}
-
-// direct classes: 0: band <= 8 bins (F=8), 1: <= 64 (F=64), 2..5: <= 512*{1,2,4,8} (F=512)
-template <typename T, int LOGE, int NARR>
-static int launch_direct_q(const FastArgs<T>& P, int qclass, long long B, cudaStream_t st) {
-  unsigned gy = (unsigned)(B * P.n_rows);
+// direct classes: 0: band <= 8 bins (F=8), 1: <= 64 (F=64), 2..5: <= 512*{1,2,4,8} (F=512);
+// float64 has no class 5 (its band staging + tiles fit 227 KB only up to Q = 4)
+template <typename T, int NARR>
+static int launch_direct_q(const FastArgs<T>& P, int qclass, unsigned gy, cudaStream_t st) {
   switch (qclass) {
-    case 0: return launch_rows_t<T, LOGE, 3, NARR, GEN_DIRECT, 1>(P, gy, st);
-    case 1: return launch_rows_t<T, LOGE, 6, NARR, GEN_DIRECT, 1>(P, gy, st);
-    case 2: return launch_rows_t<T, LOGE, 9, NARR, GEN_DIRECT, 1>(P, gy, st);
-    case 3: return launch_rows_t<T, LOGE, 9, NARR, GEN_DIRECT, 2>(P, gy, st);
-    case 4: return launch_rows_t<T, LOGE, 9, NARR, GEN_DIRECT, 4>(P, gy, st);
-    default: return launch_rows_t<T, LOGE, 9, NARR, GEN_DIRECT, 8>(P, gy, st);
+    case 0: return launch_rows<T, 3, NARR, GEN_DIRECT, 1>(P, gy, st);
+    case 1: return launch_rows<T, 6, NARR, GEN_DIRECT, 1>(P, gy, st);
+    case 2: return launch_rows<T, 9, NARR, GEN_DIRECT, 1>(P, gy, st);
+    case 3: return launch_rows<T, 9, NARR, GEN_DIRECT, 2>(P, gy, st);
+    case 4: return launch_rows<T, 9, NARR, GEN_DIRECT, 4>(P, gy, st);
+    case 5:
+      if constexpr (sizeof(T) == 4) return launch_rows<T, 9, NARR, GEN_DIRECT, 8>(P, gy, st);
+      break;
+    default: break;
   }
+  return set_error(SSQB_E_UNSUPP, "no direct row class %d", qclass);
 }
-
-template <typename T> struct DefaultLogE { static constexpr int value = sizeof(T) == 4 ? 13 : 12; };
 
 template <typename T>
-static int launch_direct(const FastArgs<T>& P, int qclass, int loge, int narr, long long B,
-                         cudaStream_t st) {
-  constexpr int LD = DefaultLogE<T>::value;
-  if (loge >= LD)
-    return narr == 2 ? launch_direct_q<T, LD, 2>(P, qclass, B, st)
-                     : launch_direct_q<T, LD, 1>(P, qclass, B, st);
-  return narr == 2 ? launch_direct_q<T, LD - 1, 2>(P, qclass, B, st)
-                   : launch_direct_q<T, LD - 1, 1>(P, qclass, B, st);
+static int launch_direct(const FastArgs<T>& P, int qclass, int narr, long long B, cudaStream_t st) {
+  const unsigned gy = (unsigned)(B * P.n_rows);
+  return narr == 2 ? launch_direct_q<T, 2>(P, qclass, gy, st) : launch_direct_q<T, 1>(P, qclass, gy, st);
 }
 
 // pass 2 of the two-pass route through the same row kernel; the scratch written by
 // pass 1 is tiled [col / R2][512][R2] with R2 = 2^P.scratch_logR2 = this kernel's lanes
 template <typename T>
 static int launch_rows_scratch(const FastArgs<T>& P, int narr, cudaStream_t st) {
-  constexpr int LD = DefaultLogE<T>::value;
-  unsigned gy = (unsigned)P.A.nrows;
-  if (P.scratch_logR2 + 9 == LD)
-    return narr == 2 ? launch_rows_t<T, LD, 9, 2, GEN_SCRATCH, 1>(P, gy, st)
-                     : launch_rows_t<T, LD, 9, 1, GEN_SCRATCH, 1>(P, gy, st);
-  if (P.scratch_logR2 + 9 == LD - 1)
-    return narr == 2 ? launch_rows_t<T, LD - 1, 9, 2, GEN_SCRATCH, 1>(P, gy, st)
-                     : launch_rows_t<T, LD - 1, 9, 1, GEN_SCRATCH, 1>(P, gy, st);
-  return set_error(SSQB_E_UNSUPP, "no row kernel for scratch tiles of 2^%d lanes", P.scratch_logR2);
+  const unsigned gy = (unsigned)P.A.nrows;
+  return narr == 2 ? launch_rows<T, 9, 2, GEN_SCRATCH, 1>(P, gy, st)
+                   : launch_rows<T, 9, 1, GEN_SCRATCH, 1>(P, gy, st);
 }
 
-static int g_p1_loge = 0, g_p1_nt = 0;       // pass-1 tile / threads (0 = default), SSQB_P1_LOGE / SSQB_P1_NT
-
-template <typename T, int LOG_M, int NARR, int LOGE1, int NT>
-static int launch_pass1f_c(const FastArgs<T>& P, cudaStream_t st, int nz = 1) {
+// pass 1 of the two-pass rows in tiles of Tile<T>::ELEMS points; gridDim.z = nz picks the
+// first array of a CTA (NARR = 1, nz = 2: W and dW in CTAs of their own)
+template <typename T, int LOG_M, int NARR>
+static int launch_pass1f_t(const FastArgs<T>& P, cudaStream_t st, int nz = 1) {
+  constexpr int LOGE1 = Tile<T>::ELEMS == 8192 ? 13 : 12;
+  constexpr int NT = Tile<T>::NT;
   constexpr int M = 1 << LOG_M;
   constexpr int R1 = (1 << LOGE1) / M;
   static_assert(R1 >= 1, "tile smaller than the transform");
   size_t smem = ((size_t)NARR * M * (R1 + 1) + M) * sizeof(cx<T>);
   auto kern = cwt_pass1f_kernel<T, LOG_M, NARR, LOGE1, NT>;
-  static size_t attr_smem = 0;
-  if (smem > attr_smem) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_smem = smem;
-  }
+  SSQB_CUDA(set_smem_limit(kern, smem));
   dim3 grid((unsigned)(512 / R1), (unsigned)P.A.nrows, (unsigned)nz);
   kern<<<grid, NT, smem, st>>>(P);
   SSQB_LAUNCH_CHECK();
   return 0;
 }
 
-// long pass-1 transforms (I2 = 1024 .. 4096): default tile; one array per CTA when two
-// do not fit the 227 KB of shared memory
+// long pass-1 transforms (I2 = 1024 .. 4096): one array per CTA when two do not fit the
+// 227 KB of shared memory
 template <typename T, int LOG_M>
 static int launch_pass1f_long(const FastArgs<T>& P, int narr, cudaStream_t st) {
-  constexpr int LD = Tile<T>::ELEMS == 8192 ? 13 : 12;
-  constexpr int NTD = Tile<T>::NT;
   constexpr int M = 1 << LOG_M;
   constexpr int R1 = Tile<T>::ELEMS / M;
   constexpr size_t two = ((size_t)2 * M * (R1 + 1) + M) * sizeof(cx<T>);
   if (narr == 2 && two <= (size_t)227 * 1024)
-    return launch_pass1f_c<T, LOG_M, 2, LD, NTD>(P, st, 1);
-  return launch_pass1f_c<T, LOG_M, 1, LD, NTD>(P, st, narr);
-}
-
-template <typename T, int LOG_M, int NARR>
-static int launch_pass1f_t(const FastArgs<T>& P, cudaStream_t st) {
-  constexpr int LD = Tile<T>::ELEMS == 8192 ? 13 : 12;
-  constexpr int NTD = Tile<T>::NT;
-  if (sizeof(T) == 4 && LOG_M <= 9) {
-    // float32 variants (tile, threads): (13,512) default, (13,1024), (12,256), (12,512)
-    int le = g_p1_loge ? g_p1_loge : LD, nt = g_p1_nt ? g_p1_nt : NTD;
-    if (le == 12 && nt == 512) return launch_pass1f_c<T, LOG_M, NARR, 12, 512>(P, st);
-    if (le == 12 && nt == 256) return launch_pass1f_c<T, LOG_M, NARR, 12, 256>(P, st);
-    if (le == 13 && nt == 1024) return launch_pass1f_c<T, LOG_M, NARR, 13, 1024>(P, st);
-  }
-  return launch_pass1f_c<T, LOG_M, NARR, LD, NTD>(P, st);
+    return launch_pass1f_t<T, LOG_M, 2>(P, st, 1);
+  return launch_pass1f_t<T, LOG_M, 1>(P, st, narr);
 }
 
 template <typename T>
@@ -222,27 +174,22 @@ static int launch_pass1v(const FastArgs<T>& P, cudaStream_t st) {
   using V4 = typename V4T<T>::type;
   size_t smem = (size_t)512 * R1 * sizeof(V4) + 512 * sizeof(cx<T>);
   auto kern = cwt_pass1v_kernel<T, R1>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
+  SSQB_CUDA(set_smem_limit(kern, smem));
   kern<<<dim3(512 / R1, (unsigned)P.A.nrows), 64 * R1, smem, st>>>(P);
   SSQB_LAUNCH_CHECK();
   return 0;
 }
 
-static int g_p1v = 1;          // SSQB_P1V=0: the older pass-1 kernel for 512-point transforms
-
 // returns -100 when this geometry has no fast pass 1 (caller uses the generic kernel)
 template <typename T>
 static int launch_pass1f(const FastArgs<T>& P, int narr, cudaStream_t st) {
-  if (P.A.logI2 == 9 && narr == 2 && g_p1v) return launch_pass1v<T>(P, st);
   switch (P.A.logI2) {
 #define SSQB_P1F(L) case L: return narr == 2 ? launch_pass1f_t<T, L, 2>(P, st) \
                                              : launch_pass1f_t<T, L, 1>(P, st);
-    SSQB_P1F(4) SSQB_P1F(5) SSQB_P1F(6) SSQB_P1F(7) SSQB_P1F(8) SSQB_P1F(9)
+    SSQB_P1F(4) SSQB_P1F(5) SSQB_P1F(6) SSQB_P1F(7) SSQB_P1F(8)
 #undef SSQB_P1F
+    // 512-point transforms of W and dW: both arrays as one 16-byte element
+    case 9: return narr == 2 ? launch_pass1v<T>(P, st) : launch_pass1f_t<T, 9, 1>(P, st);
     case 10: return launch_pass1f_long<T, 10>(P, narr, st);
     case 11: return launch_pass1f_long<T, 11>(P, narr, st);
     case 12: return launch_pass1f_long<T, 12>(P, narr, st);
@@ -257,11 +204,7 @@ static int launch_sblk_fwd(const SblkArgs<T>& S, cudaStream_t st) {
   constexpr int LP = SblkGeom<T>::LOG_P;
   size_t smem = ((size_t)1 << LP) * sizeof(cx<T>);
   auto kern = sblk_fwd_kernel<T, LP>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
+  SSQB_CUDA(set_smem_limit(kern, smem));
   kern<<<dim3((unsigned)S.nblk, (unsigned)S.B), (1 << LP) / 8, smem, st>>>(S);
   SSQB_LAUNCH_CHECK();
   return 0;
@@ -272,17 +215,13 @@ static int launch_sblk_rows_t(const SblkArgs<T>& S, cudaStream_t st) {
   using V4 = typename V4T<T>::type;
   size_t smem = ((size_t)1 << LP) * (sizeof(V4) + sizeof(cx<T>));
   auto kern = sblk_rows_kernel<T, LP, NARR, SSQ>;
-  static bool attr_set = false;
-  static int ctas = 2 * 148;
-  if (!attr_set) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int dev = 0, sms = 148, per = 2;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, kern, (1 << LP) / 8, smem) != cudaSuccess || per < 1) per = 1;
-    ctas = sms * per;
-    attr_set = true;
-  }
+  SSQB_CUDA(set_smem_limit(kern, smem));
+  // persistent grid: as many CTAs as the current device holds at once
+  int dev = 0, sms = 0, per = 0;
+  SSQB_CUDA(cudaGetDevice(&dev));
+  SSQB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  SSQB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, kern, (1 << LP) / 8, smem));
+  const long long ctas = (long long)sms * (per < 1 ? 1 : per);
   long long items = S.B * (long long)S.n_rows * S.nblk;
   unsigned g = (unsigned)(items < ctas ? items : ctas);
   if (g < 1) return 0;
@@ -335,11 +274,7 @@ static int launch_grid_dec_t(const GridArgs<T>& G, const GridRow* rows, int n_cl
   size_t smem = ((size_t)2 * Geo::M * Geo::R + Geo::M) * sizeof(cx<T>);
   if (smem > (size_t)227 * 1024) return set_error(SSQB_E_UNSUPP, "coarse grid 2^%d too long", LOG_M);
   auto kern = grid_dec_ifft_kernel<T, LOG_M>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
+  SSQB_CUDA(set_smem_limit(kern, smem));
   long long pairs = (long long)n_cls * G.B;
   dim3 grid((unsigned)((pairs + Geo::R - 1) / Geo::R));
   kern<<<grid, Geo::NT, smem, st>>>(G, rows, n_cls);
@@ -350,11 +285,7 @@ template <typename T, int LOG_M>
 static int launch_grid_dec_single(const GridArgs<T>& G, const GridRow* rows, int n_cls, cudaStream_t st) {
   size_t smem = ((size_t)1 << LOG_M) * sizeof(cx<T>);
   auto kern = grid_dec_single_kernel<T, LOG_M>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
+  SSQB_CUDA(set_smem_limit(kern, smem));
   kern<<<dim3((unsigned)(n_cls * G.B), 2), 1024, smem, st>>>(G, rows, n_cls);
   SSQB_LAUNCH_CHECK();
   return 0;
@@ -365,11 +296,7 @@ static int launch_grid_dec_split(const GridArgs<T>& G, int logR, const GridRow* 
                                  cudaStream_t st) {
   size_t smem = ((size_t)1 << LOG_MB) * sizeof(cx<T>);
   auto kern = grid_dec_split_kernel<T, LOG_MB>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
+  SSQB_CUDA(set_smem_limit(kern, smem));
   kern<<<dim3((unsigned)(((long long)n_cls * G.B) << logR), 2), 1024, smem, st>>>(G, rows, n_cls, logR);
   SSQB_LAUNCH_CHECK();
   return 0;
@@ -380,15 +307,8 @@ static int launch_grid_dec(const GridArgs<T>& G, int logM, const GridRow* rows, 
                            cudaStream_t st) {
   constexpr int BASE = (sizeof(T) == 4) ? 14 : 13;
   if (logM > BASE) return launch_grid_dec_split<T, BASE>(G, logM - BASE, rows, n_cls, st);
-  if (logM == BASE) {
-    // one CTA per transform of 2^BASE points fills an SM's shared memory (1 CTA / SM); as two CTAs
-    // of half the length (first DIF stage while reading the band) two fit an SM  (SSQB_DEC_SPLIT=0|1)
-    static int split = -1;
-    if (split < 0) { const char* e = getenv("SSQB_DEC_SPLIT"); split = e ? atoi(e) : 0; }
-    if constexpr (sizeof(T) == 4)            // float64: 2^12 points are too few for the 1024-thread kernel
-      if (split) return launch_grid_dec_split<T, BASE - 1>(G, 1, rows, n_cls, st);
-    return launch_grid_dec_single<T, BASE>(G, rows, n_cls, st);
-  }
+  // one CTA per transform of 2^BASE points (it fills an SM's shared memory)
+  if (logM == BASE) return launch_grid_dec_single<T, BASE>(G, rows, n_cls, st);
   switch (logM) {
 #define SSQB_GD(L) case L: return launch_grid_dec_t<T, L>(G, rows, n_cls, st);
     SSQB_GD(6) SSQB_GD(7) SSQB_GD(8) SSQB_GD(9) SSQB_GD(10) SSQB_GD(11) SSQB_GD(12)
@@ -405,57 +325,33 @@ template <typename T>
 static int launch_grid_dec_small(const GridArgs<T>& G, const DecSmallPlan& P, cudaStream_t st) {
   size_t smem = ((size_t)2 * 2048 + 2048) * sizeof(cx<T>);
   auto kern = grid_dec_ifft_small_kernel<T>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
+  SSQB_CUDA(set_smem_limit(kern, smem));
   if (P.cta_start[6] <= 0) return 0;
   kern<<<dim3((unsigned)P.cta_start[6]), 256, smem, st>>>(G, P);
   SSQB_LAUNCH_CHECK();
   return 0;
 }
 
-template <typename T> struct GridTaps;            // kernel width K, outputs per thread = K * PPK
-template <> struct GridTaps<float>  { static constexpr int K = 8,  PPK = 4; };
-template <> struct GridTaps<double> { static constexpr int K = 14, PPK = 2; };
+template <typename T> struct GridTaps;            // kernel width K
+template <> struct GridTaps<float>  { static constexpr int K = 8; };
+template <> struct GridTaps<double> { static constexpr int K = 14; };
 
-// outputs per thread of the float32 ssq kernel: K * interp_ppk (SSQB_INTERP_PPK=4|8)
-static int g_interp_ppk = -1;
-template <typename T> static int interp_ppk(bool ssq, int narr) {
-  if (sizeof(T) == 4 && ssq && narr == 2) {
-    if (g_interp_ppk < 0) {
-      // measured (B = 64, groups of 8): PPK = 4: 17.78 ms / step, PPK = 8: 16.74, PPK = 16: 16.49 -- a CTA's fixed cost (TMA
-      // window, modulation table, kernel values) is amortised over twice the outputs
-      const char* e = getenv("SSQB_INTERP_PPK");
-      const int v = e ? atoi(e) : 16;
-      g_interp_ppk = (v == 4 || v == 8) ? v : 16;
-    }
-    return g_interp_ppk;
-  }
-  if (sizeof(T) == 8 && ssq && narr == 2) {
-    static int ppk64 = -1;                  // float64: SSQB_INTERP_PPK64=2|4
-    if (ppk64 < 0) {
-      const char* e = getenv("SSQB_INTERP_PPK64"); ppk64 = (e && atoi(e) == 2) ? 2 : 4;   // C5: 22.80 -> 21.89 ms / 2 signals
-      const char* r = getenv("SSQB_F64_REGWIN"); if (r && atoi(r) == 0) ppk64 = 2;   // that variant is PPK = 2 only
-    }
-    return ppk64;
-  }
-  return GridTaps<T>::PPK;
+// outputs per thread of the interpolation kernel: K * interp_ppk.  ssq in float32: 16 (measured,
+// B = 64, groups of 8: PPK = 4: 17.78 ms / step, 8: 16.74, 16: 16.49 -- a CTA's fixed cost (TMA
+// window, modulation table, kernel values) is amortised over more outputs); ssq in float64: 4
+// (C5: 22.80 -> 21.89 ms / 2 signals against 2)
+template <typename T> constexpr int interp_ppk(bool ssq) {
+  return sizeof(T) == 4 ? (ssq ? 16 : 4) : (ssq ? 4 : 2);
 }
 
-template <typename T, int NARR, bool SSQ, bool RW, int PPK = GridTaps<T>::PPK>
+template <typename T, int NARR, bool SSQ>
 static int launch_grid_interp_t(const GridArgs<T>& G, unsigned max_tiles, cudaStream_t st) {
-  constexpr int K = GridTaps<T>::K, PP = K * PPK;
+  constexpr int K = GridTaps<T>::K, PPK = interp_ppk<T>(SSQ), PP = K * PPK;
   using V4 = typename V4T<T>::type;
   // coarse samples per CTA = (256 / min(U, 256)) * PP; U >= 16
   size_t smem = (size_t)(16 * PP + K - 1) * sizeof(V4) + (size_t)16 * PP * sizeof(cx<T>);
-  auto kern = grid_interp_kernel<T, K, PPK, NARR, SSQ, RW>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
+  auto kern = grid_interp_kernel<T, K, PPK, NARR, SSQ>;
+  SSQB_CUDA(set_smem_limit(kern, smem));
   dim3 grid(max_tiles, (unsigned)(G.B * G.n_rows));
   kern<<<grid, 256, smem, st>>>(G);
   SSQB_LAUNCH_CHECK();
@@ -463,29 +359,9 @@ static int launch_grid_interp_t(const GridArgs<T>& G, unsigned max_tiles, cudaSt
 }
 template <typename T>
 static int launch_grid_interp(const GridArgs<T>& G, int narr, unsigned max_tiles, cudaStream_t st) {
-  if constexpr (sizeof(T) == 8) {
-    // float64: the register window (14 x 4 doubles) against taps from shared memory
-    static int regwin = -1;
-    if (regwin < 0) { const char* e = getenv("SSQB_F64_REGWIN"); regwin = e ? atoi(e) : 1; }
-    if (!regwin) {
-      if (narr == 2 && G.ssq) return launch_grid_interp_t<T, 2, true, false>(G, max_tiles, st);
-      if (narr == 2) return launch_grid_interp_t<T, 2, false, false>(G, max_tiles, st);
-      return launch_grid_interp_t<T, 1, false, false>(G, max_tiles, st);
-    }
-  }
-  if (narr == 2 && G.ssq) {
-    if constexpr (sizeof(T) == 4)
-      switch (interp_ppk<T>(true, 2)) {
-        case 8:  return launch_grid_interp_t<T, 2, true, true, 8>(G, max_tiles, st);
-        case 16: return launch_grid_interp_t<T, 2, true, true, 16>(G, max_tiles, st);
-        default: break;
-      }
-    if constexpr (sizeof(T) == 8)
-      if (interp_ppk<T>(true, 2) == 4) return launch_grid_interp_t<T, 2, true, true, 4>(G, max_tiles, st);
-    return launch_grid_interp_t<T, 2, true, true>(G, max_tiles, st);
-  }
-  if (narr == 2) return launch_grid_interp_t<T, 2, false, true>(G, max_tiles, st);
-  return launch_grid_interp_t<T, 1, false, true>(G, max_tiles, st);
+  if (narr == 2 && G.ssq) return launch_grid_interp_t<T, 2, true>(G, max_tiles, st);
+  if (narr == 2) return launch_grid_interp_t<T, 2, false>(G, max_tiles, st);
+  return launch_grid_interp_t<T, 1, false>(G, max_tiles, st);
 }
 
 
@@ -504,11 +380,16 @@ struct CwtPlan : public CwtPlanBase {
   bool have_grid = false;
   // scratch of the two-pass route.  The path is issue-bound, not HBM-bound, so a
   // scratch larger than L2 (fewer, fuller launches) beats an L2-resident one.
-  size_t scratch_bytes = (size_t)512 << 20;
+  static constexpr size_t SCRATCH_BYTES = (size_t)512 << 20;
+  // route switches, read from the environment once per plan (init): a route that is off leaves
+  // its rows to the next one, which is how tests reach the direct, block and two-pass rows at
+  // shapes where the default routes claim every row
+  struct Routes {
+    bool fast, grid, sblk, block;     // SSQB_NO_FAST / _NO_GRID / _NO_SBLK / _NO_BLOCK = 1: off
+    int grid_max_logm;                // SSQB_GRID_MAX_LOGM: longest coarse grid (0: no cap)
+  } routes{};
   // fast path (n_up >= 2^13, device-evaluated wavelets): band tables + row classes
   bool fast = false;
-  int loge = 13;
-  int scratch_loge = 12;                // two-pass route: pass-2 tile = 2^scratch_loge points
   DevBuf<long long> tab_off_d;
   DevBuf<T> tab_p_d, tab_pd_d;
   static constexpr int NCLS = 6;          // band <= 8, 64, 512, 1024, 2048, 4096 bins
@@ -522,7 +403,7 @@ struct CwtPlan : public CwtPlanBase {
   // blocks of P = 2^logP samples with a halo of h2 samples on each side
   static constexpr int BLK_NCLS = 5;
   struct BlockClass {
-    int logP = 13, h2 = 0, hop = 0, nblk = 0, log_lo = 7, loge = 13;
+    int logP = 13, h2 = 0, hop = 0, nblk = 0, log_lo = 7;
     DevBuf<RowInfo> rows[4];                  // Q <= 1, 2, 4, 8 on the block grid
     int n_rows[4] = {0, 0, 0, 0};
     DevBuf<long long> row_n1;                 // [B*nblk] per-block left pad for the loader
@@ -581,9 +462,7 @@ struct CwtPlan : public CwtPlanBase {
   static constexpr int NLANES = 3;
   cudaStream_t lanes[NLANES] = {nullptr, nullptr, nullptr};
   cudaEvent_t ev_lane_fork = nullptr, ev_lane_done[NLANES] = {nullptr, nullptr, nullptr};
-  int use_lanes = 1;
   ~CwtPlan() {
-    if (gexec) cudaGraphExecDestroy(gexec);
     for (int i = 0; i < NLANES; ++i) {
       if (ev_lane_done[i]) cudaEventDestroy(ev_lane_done[i]);
       if (lanes[i]) cudaStreamDestroy(lanes[i]);
@@ -620,7 +499,6 @@ struct CwtPlan : public CwtPlanBase {
     return 0;
   }
   int set_profiling(int on) override {
-    drop_graph();
     for (auto e : ev) cudaEventDestroy(e);
     ev.clear(); ev_kind.clear(); ev_rows.clear();
     profiling = on != 0;
@@ -658,9 +536,9 @@ struct CwtPlan : public CwtPlanBase {
     logI2 = logn - logF;
     if (logI2 < 1) { logI2 = 1; logF = logn - 1; }
     log_lo = (logn + 1) / 2;
-    if (const char* e = getenv("SSQB_SCRATCH_MB")) {
-      long v = atol(e); if (v > 0) scratch_bytes = (size_t)v << 20;
-    }
+    auto env = [](const char* name) { const char* e = getenv(name); return e ? atoi(e) : 0; };
+    routes = Routes{!env("SSQB_NO_FAST"), !env("SSQB_NO_GRID"), !env("SSQB_NO_SBLK"),
+                    !env("SSQB_NO_BLOCK"), env("SSQB_GRID_MAX_LOGM")};
     std::vector<T> sc((size_t)d.na);
     std::vector<long long> lo((size_t)d.na), len((size_t)d.na);
     for (int a = 0; a < d.na; ++a) {
@@ -685,47 +563,22 @@ struct CwtPlan : public CwtPlanBase {
       SSQB_CUDA(cudaStreamCreateWithFlags(&lanes[i], cudaStreamNonBlocking));
       SSQB_CUDA(cudaEventCreateWithFlags(&ev_lane_done[i], cudaEventDisableTiming));
     }
-    if (const char* e = getenv("SSQB_LANES")) use_lanes = atoi(e);
     return init_fast(lo, len);
   }
 
   int init_fast(const std::vector<long long>& lo, const std::vector<long long>& len) {
     fast = false; have_blocks = false;
-    if (const char* e = getenv("SSQB_NO_FAST")) { if (atoi(e)) return 0; }
+    if (!routes.fast) return 0;
     if (logF != 9 || logI2 < 4 || d.wavelet == SSQB_WAV_TABLE) return 0;
-    loge = 12;                       // direct rows: 4096-point tiles (R2 = 8), 2 CTAs / SM
-    if (const char* e = getenv("SSQB_LOGE")) { int v = atoi(e); if (v >= 11 && v <= 13) loge = v; }
-    scratch_loge = 12;
-    if (const char* e = getenv("SSQB_SCRATCH_LOGE")) {
-      int v = atoi(e); if (v == DefaultLogE<T>::value || v == DefaultLogE<T>::value - 1) scratch_loge = v;
-    }
-    if (logI2 < scratch_loge - 9) scratch_loge = 9 + logI2;       // tile lanes <= I2
-    if (logI2 > 12) scratch_loge = DefaultLogE<T>::value;   // generic pass 1 tiling
-    if (const char* e = getenv("SSQB_P1V")) g_p1v = atoi(e);
-    if (const char* e = getenv("SSQB_P1_LOGE")) g_p1_loge = atoi(e);
-    if (const char* e = getenv("SSQB_P1_NT")) g_p1_nt = atoi(e);
-    if (const char* e = getenv("SSQB_BPT")) { int v = atoi(e); if (v == 1 || v == 2) g_rows_bpt = v; }
-    if (sizeof(T) == 8 && loge > 12) loge = 12;
     // float64 staging (32 B per band bin) + 128 KB of tiles must fit 227 KB: Q <= 4
-    int qmax_direct = (sizeof(T) == 4) ? 8 : 4;
-    if (const char* e = getenv("SSQB_QMAX")) {
-      int v = atoi(e); if (v >= 0 && v <= qmax_direct) qmax_direct = v;
-    }
-    int adaptive = 1;
-    if (const char* e = getenv("SSQB_ADAPTIVE_F")) adaptive = atoi(e);
-    int use_blocks = (d.tsupport_host != nullptr) ? 1 : 0;
-    if (const char* e = getenv("SSQB_NO_BLOCK")) { if (atoi(e)) use_blocks = 0; }
-    int blk_loge = 12;
-    if (const char* e = getenv("SSQB_BLK_LOGE")) { int v = atoi(e); if (v == 12 || v == 13) blk_loge = v; }
+    constexpr int qmax_direct = (sizeof(T) == 4) ? 8 : 4;
+    const bool use_blocks = d.tsupport_host != nullptr && routes.block;
     // short blocks: the signal must be a few blocks long, and every halo must stay inside the
     // padding the reference adds (the block loader extends the signal by the padding rule)
-    int use_sblk = use_blocks;
-    if (const char* e = getenv("SSQB_NO_SBLK")) { if (atoi(e)) use_sblk = 0; }
-    if (logn < SBLK_LOGP + 2 || d.n1 < 512 || d.n_up - d.n1 - d.N < 512) use_sblk = 0;
+    bool use_sblk = use_blocks && routes.sblk;
+    if (logn < SBLK_LOGP + 2 || d.n1 < 512 || d.n_up - d.n1 - d.N < 512) use_sblk = false;
     for (int c = 0; c < SBLK_NCLS; ++c) sblk[c].rows.clear();
     have_sblk = false; have_cut = false;
-    int sblk_smooth = 1;                       // SSQB_SBLK_SMOOTH=0: only the Nyquist-cut rows
-    if (const char* e = getenv("SSQB_SBLK_SMOOTH")) sblk_smooth = atoi(e);
 
     // ---- route every scale: block class / direct class / two-pass --------------------
     // block length 2^logP with a halo of h2 samples each side; the two long classes only
@@ -753,8 +606,8 @@ struct CwtPlan : public CwtPlanBase {
       if (use_sblk && q >= 2 && len[a] < d.n_up) {
         const long long S = d.tsupport_host[a];
         int sc = -1;
-        if (S > 0 && S <= 512 && sblk_smooth) sc = 0;
-        else if (S > 512 && S <= 1024 && sizeof(T) == 4 && sblk_smooth) sc = 1;
+        if (S > 0 && S <= 512) sc = 0;
+        else if (S > 512 && S <= 1024 && sizeof(T) == 4) sc = 1;
         else if (S < 0 && d.wavelet != SSQB_WAV_TABLE && lo[a] >= 0 &&
                  lo[a] + len[a] - 1 == d.n_up / 2 && (-S) + 2 * SBLK_TAPER_HALF <= 512) sc = 2;
         if (sc >= 0) {
@@ -791,7 +644,7 @@ struct CwtPlan : public CwtPlanBase {
       if (routed) { big_scales_all.push_back(a); continue; }   // two-pass when blocks are off
       if (q > qmax_direct) { big_scales.push_back(a); big_scales_all.push_back(a); continue; }
       int c = q <= 1 ? 2 : q <= 2 ? 3 : q <= 4 ? 4 : 5;
-      if (adaptive) { if (len[a] <= 8) c = 0; else if (len[a] <= 64) c = 1; }
+      if (len[a] <= 8) c = 0; else if (len[a] <= 64) c = 1;
       cls[c].push_back(a);
     }
     SSQB_CUDA(tab_off_d.upload(off));
@@ -821,7 +674,6 @@ struct CwtPlan : public CwtPlanBase {
       K.logP = logPs[c]; K.h2 = h2s[c]; K.hop = (1 << K.logP) - 2 * K.h2;
       K.nblk = (int)((d.N + K.hop - 1) / K.hop);
       K.log_lo = (K.logP + 1) / 2;
-      K.loge = (K.logP - 9 >= blk_loge - 9) ? blk_loge : 9 + (K.logP - 9);
       for (int k = 0; k < 4; ++k)
         if (K.n_rows[k]) SSQB_CUDA(K.rows[k].upload(blists[c][k]));
       const long long Pn = 1ll << K.logP;
@@ -942,13 +794,11 @@ struct CwtPlan : public CwtPlanBase {
                 std::vector<char>& is_grid) {
     have_grid_rows = false; grid_rows.clear(); grid_v_total = 0;
     for (int l = 0; l < 20; ++l) { grid_cls_first[l] = 0; grid_cls_n[l] = 0; }
-    if (const char* e = getenv("SSQB_NO_GRID")) { if (atoi(e)) return 0; }
-    if (logn < 13) return 0;
+    if (!routes.grid || logn < 13) return 0;
     int max_logm = GRID_MAX_LOGM;
     if (max_logm > logn - 4) max_logm = logn - 4;          // U = n/M >= 16
-    if (const char* e = getenv("SSQB_GRID_MAX_LOGM")) {
-      int v = atoi(e); if (v >= GRID_MIN_LOGM && v < max_logm) max_logm = v;
-    }
+    const int v = routes.grid_max_logm;
+    if (v >= GRID_MIN_LOGM && v < max_logm) max_logm = v;
     std::vector<GridRow> rows;
     for (int a = 0; a < d.na; ++a) {
       const long long L = len[a];
@@ -1090,7 +940,7 @@ struct CwtPlan : public CwtPlanBase {
     return prof_end(st);
   }
   int grid_stage_b(const GridArgs<T>& G, long long B, int narr, cudaStream_t st) {
-    const int PP = GridTaps<T>::K * interp_ppk<T>(G.ssq != 0, narr);
+    const int PP = GridTaps<T>::K * interp_ppk<T>(G.ssq != 0);
     unsigned max_tiles = 1;                               // tiles of the widest row class
     for (int lm = GRID_MIN_LOGM; lm <= GRID_MAX_LOGM; ++lm) {
       if (!grid_cls_n[lm]) continue;
@@ -1152,27 +1002,26 @@ struct CwtPlan : public CwtPlanBase {
     std::vector<double> c(r->cst_host, r->cst_host + d.na);
     SSQB_CUDA(cst_d.upload(c));
     have_grid = true;
-    drop_graph();                 // kernel arguments (grid, const) are baked into a graph
     return 0;
   }
 
   // rows of G that fit the scratch budget
   long long rows_per_chunk(int narr, long long total_rows) {
     size_t per_row = (size_t)narr * (size_t)d.n_up * sizeof(cx<T>);
-    long long r = (long long)(scratch_bytes / per_row);
+    long long r = (long long)(SCRATCH_BYTES / per_row);
     if (r < 1) r = 1;
     if (r > total_rows) r = total_rows;
     return r;
   }
   cudaError_t ensure_scratch(int narr, long long rows) {
-    long long E = fast ? (1ll << scratch_loge) : (long long)Tile<T>::ELEMS;
+    long long E = fast ? (1ll << ROWS_LOGE) : (long long)Tile<T>::ELEMS;
     long long R2 = E >> logF;
     long long ncols = rows << logI2;
     long long tiles = (ncols + R2 - 1) / R2;
     return G_d.ensure((size_t)narr * (size_t)tiles * (size_t)E);
   }
   long long arr_stride(long long rows) {
-    long long E = fast ? (1ll << scratch_loge) : (long long)Tile<T>::ELEMS;
+    long long E = fast ? (1ll << ROWS_LOGE) : (long long)Tile<T>::ELEMS;
     long long R2 = E >> logF;
     long long ncols = rows << logI2;
     return ((ncols + R2 - 1) / R2) * E;
@@ -1193,78 +1042,6 @@ struct CwtPlan : public CwtPlanBase {
     }
     return 0;
   }
-
-  // ---- CUDA-graph replay of a repeated call (same buffers, same batch) ------------------
-  // A step is ~26 short launches on two streams; when the very same call is issued again
-  // (a streaming / benchmark loop re-using its buffers) the launch sequence is captured
-  // once and replayed with one cudaGraphLaunch.  Single-slot cache; any change of
-  // pointers, batch, flags or reassignment parameters falls back to plain launches.
-  struct GraphKey {
-    const void *x = nullptr, *Wx = nullptr, *dWx = nullptr, *Tx = nullptr;
-    long long B = 0; int ssq = 0, rpadded = 0;
-    bool operator==(const GraphKey& o) const {
-      return x == o.x && Wx == o.Wx && dWx == o.dWx && Tx == o.Tx && B == o.B &&
-             ssq == o.ssq && rpadded == o.rpadded;
-    }
-  };
-  GraphKey last_key, graph_key;
-  int key_hits = 0;
-  cudaGraphExec_t gexec = nullptr;
-  bool graphs_ok = true;
-  void drop_graph() {
-    if (gexec) { cudaGraphExecDestroy(gexec); gexec = nullptr; }
-    key_hits = 0; last_key = GraphKey();
-  }
-
-  int exec(const void* xv, long long B, void* Wxv, void* dWxv, void* Txv, bool ssq,
-           const double* out_mul_host, bool rpadded, cudaStream_t st) override {
-    static int env_graph = -1;
-    if (env_graph < 0) { const char* e = getenv("SSQB_GRAPH"); env_graph = e ? atoi(e) : 0; }
-    if (!env_graph || !graphs_ok || profiling || out_mul_host || !fast)
-      return exec_impl(xv, B, Wxv, dWxv, Txv, ssq, out_mul_host, rpadded, st);
-    GraphKey k; k.x = xv; k.Wx = Wxv; k.dWx = dWxv; k.Tx = Txv; k.B = B;
-    k.ssq = ssq; k.rpadded = rpadded;
-    if (gexec && k == graph_key) {
-      SSQB_CUDA(cudaGraphLaunch(gexec, st));
-      g_launch_count.fetch_add(graph_launches, std::memory_order_relaxed);
-      return 0;
-    }
-    if (!(k == last_key)) { last_key = k; key_hits = 1; }
-    else ++key_hits;
-    if (key_hits < 3) return exec_impl(xv, B, Wxv, dWxv, Txv, ssq, out_mul_host, rpadded, st);
-    // third identical call in a row: every buffer exists by now -> capture
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    cudaStreamIsCapturing(st, &cs);
-    if (cs != cudaStreamCaptureStatusNone)            // caller is capturing already
-      return exec_impl(xv, B, Wxv, dWxv, Txv, ssq, out_mul_host, rpadded, st);
-    if (gexec) { cudaGraphExecDestroy(gexec); gexec = nullptr; }
-    long long l0 = g_launch_count.load();
-    if (cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
-      cudaGetLastError(); graphs_ok = false;
-      return exec_impl(xv, B, Wxv, dWxv, Txv, ssq, out_mul_host, rpadded, st);
-    }
-    int rc = exec_impl(xv, B, Wxv, dWxv, Txv, ssq, out_mul_host, rpadded, st);
-    cudaGraph_t g = nullptr;
-    cudaError_t e = cudaStreamEndCapture(st, &g);
-    graph_launches = g_launch_count.load() - l0;
-    g_launch_count.fetch_sub(graph_launches, std::memory_order_relaxed);   // nothing ran yet
-    if (rc != 0 || e != cudaSuccess || !g) {
-      cudaGetLastError(); if (g) cudaGraphDestroy(g);
-      graphs_ok = false;
-      return exec_impl(xv, B, Wxv, dWxv, Txv, ssq, out_mul_host, rpadded, st);
-    }
-    e = cudaGraphInstantiate(&gexec, g, 0);
-    cudaGraphDestroy(g);
-    if (e != cudaSuccess) {
-      cudaGetLastError(); gexec = nullptr; graphs_ok = false;
-      return exec_impl(xv, B, Wxv, dWxv, Txv, ssq, out_mul_host, rpadded, st);
-    }
-    graph_key = k;
-    SSQB_CUDA(cudaGraphLaunch(gexec, st));
-    g_launch_count.fetch_add(graph_launches, std::memory_order_relaxed);
-    return 0;
-  }
-  long long graph_launches = 0;
 
   // Calls on one plan share its scratch, tables and worker streams, so consecutive calls are
   // ordered on the device whatever streams they arrive on: each call first waits for the
@@ -1306,8 +1083,8 @@ struct CwtPlan : public CwtPlanBase {
     return S;
   }
 
-  int exec_impl(const void* xv, long long B, void* Wxv, void* dWxv, void* Txv, bool ssq,
-                const double* out_mul_host, bool rpadded, cudaStream_t st) {
+  int exec(const void* xv, long long B, void* Wxv, void* dWxv, void* Txv, bool ssq,
+           const double* out_mul_host, bool rpadded, cudaStream_t st) override {
     if (!ev_done) SSQB_CUDA(cudaEventCreateWithFlags(&ev_done, cudaEventDisableTiming));
     if (ev_done_valid) SSQB_CUDA(cudaStreamWaitEvent(st, ev_done, 0));
     const long long S = (B >= 1) ? group_size(B, ssq, rpadded) : B;
@@ -1372,9 +1149,10 @@ struct CwtPlan : public CwtPlanBase {
       if (ssq && zero_self_) {                // later groups were zeroed by the previous group's kernels
         const size_t bytes = (size_t)total_rows * (size_t)Nout * sizeof(cx<T>);   // multiple of 8
         const size_t n16 = bytes / 16;
-        static int zctas = -1;                 // CTAs per SM of the zero fill (SSQB_ZERO_CTAS)
-        if (zctas < 0) { const char* e = getenv("SSQB_ZERO_CTAS"); zctas = e ? atoi(e) : 16; if (zctas < 1) zctas = 1; }
-        size_t nb = (n16 + 255) / 256; if (nb > (size_t)148 * zctas) nb = (size_t)148 * zctas; if (nb < 1) nb = 1;
+        int dev = 0, sms = 0;                  // at most 16 CTAs per SM of the current device
+        SSQB_CUDA(cudaGetDevice(&dev));
+        SSQB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+        size_t nb = (n16 + 255) / 256; if (nb > (size_t)sms * 16) nb = (size_t)sms * 16; if (nb < 1) nb = 1;
         zero_fill_kernel<<<(unsigned)nb, 256, 0, side>>>(reinterpret_cast<uint4*>(Tx), n16,
                                                         reinterpret_cast<unsigned char*>(Tx) + n16 * 16,
                                                         (int)(bytes - n16 * 16));
@@ -1416,7 +1194,7 @@ struct CwtPlan : public CwtPlanBase {
     //   * the spectrum xh (forward FFT, main stream)         -> direct and two-pass rows
     //   * the block spectra + zeroed Tx (side stream, ev_join) -> block rows / any ssq row
     // so block rows can run under the forward FFT and pass 1, which leave most SMs idle.
-    const bool lanes_on = use_lanes && !profiling && fast;
+    const bool lanes_on = !profiling && fast;
     const bool side_used = need_join;
     bool lane_used[NLANES] = {false, false, false};
     bool got_join[NLANES + 1] = {false, false, false, false};
@@ -1437,7 +1215,7 @@ struct CwtPlan : public CwtPlanBase {
       for (int i = first + 1; i <= (lanes_on ? NLANES : 0); ++i) if (load[i] < load[k]) k = i;
       return k;
     };
-    struct Job { double w; FastArgs<T> P; int cls; int le; long long gb; long long rows; int sblk_cls; };
+    struct Job { double w; FastArgs<T> P; int cls; long long gb; long long rows; int sblk_cls; };
     auto run_jobs = [&](std::vector<Job>& jobs, bool need_xh, int first) -> int {
       std::sort(jobs.begin(), jobs.end(), [](const Job& a, const Job& b) { return a.w > b.w; });
       for (const Job& J : jobs) {
@@ -1456,7 +1234,7 @@ struct CwtPlan : public CwtPlanBase {
           S.write_dWx = dWx ? 1 : 0;
           r2 = launch_sblk_rows<T>(S, narr, ssq, ls);
         } else {
-          r2 = launch_direct<T>(J.P, J.cls, J.le, narr, J.gb, ls);
+          r2 = launch_direct<T>(J.P, J.cls, narr, J.gb, ls);
         }
         if (r2) return r2;
         r2 = prof_end(ls); if (r2) return r2;
@@ -1484,7 +1262,7 @@ struct CwtPlan : public CwtPlanBase {
           J.P.tab_off = K.off_d.p; J.P.tab_p = K.p_d.p; J.P.tab_pd = K.pd_d.p;
           J.P.write_dWx = dWx ? 1 : 0; J.P.ssq = ssq ? 1 : 0;
           J.P.blk_n = K.nblk; J.P.blk_hop = K.hop; J.P.blk_h2 = K.h2;
-          J.cls = 2 + k; J.le = K.loge; J.gb = vrows; J.rows = B * K.n_rows[k];
+          J.cls = 2 + k; J.gb = vrows; J.rows = B * K.n_rows[k];
           J.w = (double)J.rows * frac * qw[k]; J.sblk_cls = -1;
           bjobs.push_back(J);
         }
@@ -1492,7 +1270,7 @@ struct CwtPlan : public CwtPlanBase {
       for (int c = 0; c < SBLK_NCLS; ++c) {
         if (!sblk[c].used() || sblk[c].analytic) continue;
         Job J; memset(&J.P, 0, sizeof(J.P));
-        J.cls = 0; J.le = 0; J.gb = 0; J.rows = B * (long long)sblk[c].rows.size();
+        J.cls = 0; J.gb = 0; J.rows = B * (long long)sblk[c].rows.size();
         J.w = (double)J.rows * 0.8; J.sblk_cls = c;
         bjobs.push_back(J);
       }
@@ -1556,7 +1334,7 @@ struct CwtPlan : public CwtPlanBase {
         P.A = A; P.rowinfo = nullptr; P.n_rows = 0;
         P.tab_off = tab_off_d.p; P.tab_p = tab_p_d.p; P.tab_pd = tab_pd_d.p;
         P.write_dWx = dWx ? 1 : 0; P.ssq = ssq ? 1 : 0;
-        P.scratch_logR2 = scratch_loge - 9;
+        P.scratch_logR2 = ROWS_LOGE - 9;
         rc = prof_begin(1, nr, ts); if (rc) return rc;
         rc = fast ? launch_pass1f<T>(P, narr, ts) : -100;
         if (rc == -100) rc = launch_pass1<T, MODE_CWT>(A, narr, ts);
@@ -1588,13 +1366,13 @@ struct CwtPlan : public CwtPlanBase {
         J.P.rowinfo = qrows_d[c].p; J.P.n_rows = n_qrows[c];
         J.P.tab_off = tab_off_d.p; J.P.tab_p = tab_p_d.p; J.P.tab_pd = tab_pd_d.p;
         J.P.write_dWx = dWx ? 1 : 0; J.P.ssq = ssq ? 1 : 0; J.P.scratch_logR2 = 0;
-        J.cls = c; J.le = loge; J.gb = B; J.rows = B * n_qrows[c];
+        J.cls = c; J.gb = B; J.rows = B * n_qrows[c];
         J.w = (double)J.rows * cw[c]; J.sblk_cls = -1;
         jobs.push_back(J);
       }
       if (use_cut) {
         Job J; memset(&J.P, 0, sizeof(J.P));
-        J.cls = 0; J.le = 0; J.gb = 0; J.rows = B * (long long)sblk[2].rows.size();
+        J.cls = 0; J.gb = 0; J.rows = B * (long long)sblk[2].rows.size();
         J.w = (double)J.rows * 0.9; J.sblk_cls = 2;
         jobs.push_back(J);
       }
@@ -1611,7 +1389,7 @@ struct CwtPlan : public CwtPlanBase {
   }
 
   // Host buffers in, host buffers out (pinned memory recommended).  The batch is cut into
-  // chunks of `host_chunk` signals that ping-pong between two device staging slots:
+  // chunks of two signals that ping-pong between two device staging slots:
   // chunk c is transformed on the caller's stream while the copy stream still drains the
   // outputs of chunk c-1 over PCIe, so the device holds two chunks of outputs, not the batch.
   cudaStream_t copy_st = nullptr;
@@ -1619,9 +1397,7 @@ struct CwtPlan : public CwtPlanBase {
   int exec_host(const void* x, long long B, void* Wx, void* dWx, void* Tx, bool ssq,
                 const double* out_mul_host, bool rpadded, cudaStream_t st) override {
     if (B < 1) return set_error(SSQB_E_ARG, "B must be >= 1");
-    long long CH = 2;
-    if (const char* e = getenv("SSQB_HOST_CHUNK")) { long v = atol(e); if (v >= 1) CH = v; }
-    if (CH > B) CH = B;
+    const long long CH = B < 2 ? B : 2;
     const long long Nout = rpadded ? d.n_up : d.N;
     const size_t nx = (size_t)CH * (size_t)d.N, nout = (size_t)CH * d.na * (size_t)Nout;
     SSQB_CUDA(x_stage.ensure(2 * nx));

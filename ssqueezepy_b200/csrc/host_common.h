@@ -4,6 +4,8 @@
 #include <atomic>
 #include <cstdio>
 #include <cstdarg>
+#include <map>
+#include <mutex>
 #include <string>
 #include <vector>
 #include <cmath>
@@ -37,6 +39,24 @@ inline int set_error(int code, const char* fmt, ...) {
       return ::ssqb::set_error((int)_e, "kernel launch failed: %s (%s:%d)",      \
                                cudaGetErrorString(_e), __FILE__, __LINE__);      \
   } while (0)
+
+// Raises the dynamic shared-memory limit of a kernel on the current device to `bytes`, unless an
+// earlier launch there set at least that much.  The attribute belongs to the device, so a process
+// that launches on a second GPU sets it again there.
+template <typename... Args>
+inline cudaError_t set_smem_limit(void (*kern)(Args...), size_t bytes) {
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> done;    // (kernel, device) -> bytes set
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  std::lock_guard<std::mutex> lk(mu);
+  size_t& have = done[{reinterpret_cast<const void*>(kern), dev}];
+  if (bytes <= have) return cudaSuccess;
+  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e == cudaSuccess) have = bytes;
+  return e;
+}
 
 inline int ilog2_exact(long long v) {     // -1 if not a power of two
   if (v <= 0 || (v & (v - 1))) return -1;

@@ -47,12 +47,7 @@ static int launch_stft_pow2(const StftArgs<T>& A, int logm, cudaStream_t st) {
       constexpr int M = 1 << L; constexpr int R = Tile<T>::ELEMS / M;                     \
       size_t smem = ((size_t)M * (R + 1) + M) * sizeof(cx<T>);                            \
       auto kern = stft_pow2_kernel<T, L, SSQ>;                                            \
-      static bool attr_done = false;                                                      \
-      if (!attr_done) {                                                                   \
-        SSQB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                       (int)smem));                                       \
-        attr_done = true;                                                                 \
-      }                                                                                   \
+      SSQB_CUDA(set_smem_limit(kern, smem));                                              \
       kern<<<(unsigned)((total + R - 1) / R), Tile<T>::NT, smem, st>>>(A);                \
       SSQB_LAUNCH_CHECK();                                                                \
       return 0; }

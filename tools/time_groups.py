@@ -43,5 +43,5 @@ for g in groups:
         run()
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / it
-    print("B=%d group=%d zero_ctas=%s: %.3f ms/step  %.1f Msamples/s  hbm_frac %.3f"
-          % (B, g, os.environ.get('SSQB_ZERO_CTAS', '16'), ms, B * N / ms / 1e3, bytes_step / ms / 1e6 / 6572.2), flush=True)
+    print("B=%d group=%d: %.3f ms/step  %.1f Msamples/s  hbm_frac %.3f"
+          % (B, g, ms, B * N / ms / 1e3, bytes_step / ms / 1e6 / 6572.2), flush=True)
